@@ -25,6 +25,13 @@ snapshot (SURVEY.md §8d generator).
   cpu_baseline / --impl reference : the CPU restatement of the reference's per-cell path (oracle/, string
               parsing + per-cell re-summation of bound pods) on the host cores.  The Rust reference itself
               cannot be built in this image (no rustc/cargo), so kind = "port".
+
+  --dump-outputs DIR : after the timed resident steps of each workload, rank 0 writes what the last of them returned,
+              as DIR/<workload>_<name>.npy: node_idx (float32) and score (float64) of every pod of the batch (all ranks'
+              shards in pod order), feasible_count (float32) of rank 0's shard and, unless --no-mask, the feasible mask of
+              DUMP_MASK_ROWS pods of that shard (mask_rows: [rows, N] float32 0/1; mask_row_ids: their pod indices,
+              float64), rows drawn with the workload's seed.  Inputs are generated from fixed seeds, so two builds run
+              with the same arguments can be compared file by file.  About 48 MB for the default c3 + c2 run.
 """
 import argparse
 import importlib.util
@@ -46,6 +53,7 @@ METRIC = "pod_node_predicate_cells_per_sec"
 UNIT = "cells/s"
 FALLBACK_HBM_GBS = 6650.0
 PKG_DIR = os.path.join(ROOT, "kube-scheduler-rs-reference_b200")
+DUMP_MASK_ROWS = 128  # c3: 128 x 50k nodes x 4 B = 25.6 MB of the 6.25 GB mask
 
 
 def parse_args():
@@ -65,7 +73,13 @@ def parse_args():
     ap.add_argument("--no-secondary", action="store_true", help="N=1: skip the secondary c2 object")
     ap.add_argument("--no-objects", action="store_true", help="N=1: skip the object-level end-to-end figure")
     ap.add_argument("--cpu-seconds", type=float, default=12.0, help="CPU work budget of the baseline sample")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step as DIR/*.npy")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
+    return args
 
 
 def hbm_peak():
@@ -363,6 +377,35 @@ def run_workload(ks, torch, dist, args, workload, world, rank, local, steps, war
             dist.barrier()
         torch.cuda.synchronize()
 
+    def gathered_bindings():
+        """node_idx [world, cap] int32 and score [world, cap] int64 as this rank holds them after a step."""
+        if xch is not None:
+            return xch.read()
+        g = (d_all if use_nccl else d_bind).cpu().numpy().reshape(-1, cap * 12)
+        return g[:, 8 * cap:12 * cap].copy().view(np.int32), g[:, :8 * cap].copy().view(np.int64)
+
+    def shard_len(r):
+        lo_r, hi_r = ks.multigpu.shard_bounds(P_all, world, r) if strong else (0, P_all)
+        return hi_r - lo_r
+
+    def last_step_outputs():
+        """--dump-outputs: the arrays a caller of step_resident holds after it (module docstring)."""
+        g_idx, g_score = gathered_bindings()
+        out = {"node_idx": np.concatenate([g_idx[r, :shard_len(r)] for r in range(world)]),
+               "score": np.concatenate([g_score[r, :shard_len(r)] for r in range(world)]),
+               "feasible_count": d_cnt[:P].cpu().numpy().view(np.uint32)}
+        if emit_mask:
+            rows = np.sort(np.random.default_rng(seed).choice(P, size=min(P, DUMP_MASK_ROWS), replace=False))
+            picked = d_mask.index_select(0, torch.from_numpy(rows).to(dev)).cpu().numpy()
+            out["mask_rows"] = np.unpackbits(picked, axis=1, bitorder="little")[:, :N]
+            out["mask_row_ids"] = rows
+        dtypes = {"score": np.float64, "mask_row_ids": np.float64}
+        for name, a in out.items():
+            f = a.astype(dtypes.get(name, np.float32))
+            assert np.array_equal(f.astype(a.dtype), a), f"{name} is not exactly representable as {f.dtype}"
+            out[name] = f
+        return out
+
     # ---- warm-up ----
     for _ in range(max(warmup, 3)):
         step_resident(False)
@@ -401,6 +444,7 @@ def run_workload(ks, torch, dist, args, workload, world, rank, local, steps, war
     barrier()
     t_wall = time.perf_counter() - t_wall0
     launches = ks.launch_count() - launches0
+    dumped = last_step_outputs() if args.dump_outputs and rank == 0 else None
     # device-clock stamps of the last timed step (us from the first kernel of the step seen by the stamps)
     xtrace = None
     if xch is not None or os.environ.get("KS_TRACE") == "1":
@@ -465,16 +509,7 @@ def run_workload(ks, torch, dist, args, workload, world, rank, local, steps, war
     barrier()
     hb = h_bind.numpy()
     e_score, e_idx, e_cnt = hb[:8 * P].view(np.int64), hb[8 * P:12 * P].view(np.int32), hb[12 * P:16 * P].view(np.uint32)
-    if xch is not None:
-        g_idx, g_score = xch.read()
-    elif use_nccl:
-        g = d_all.cpu().numpy().reshape(world, cap * 12)
-        g_score = g[:, :8 * cap].copy().view(np.int64).reshape(world, cap)
-        g_idx = g[:, 8 * cap:12 * cap].copy().view(np.int32).reshape(world, cap)
-    else:
-        g = d_bind.cpu().numpy()
-        g_score = g[:8 * cap].view(np.int64).reshape(1, cap)
-        g_idx = g[8 * cap:12 * cap].view(np.int32).reshape(1, cap)
+    g_idx, g_score = gathered_bindings()
     assert np.array_equal(g_idx[rank, :P], e_idx) and np.array_equal(g_score[rank, :P], e_score), "resident and e2e bindings differ"
     assert np.array_equal(d_cnt.cpu().numpy()[:P].view(np.uint32), e_cnt), "resident and e2e feasible counts differ"
     assert np.array_equal(e_idx < 0, e_cnt == 0)
@@ -483,8 +518,7 @@ def run_workload(ks, torch, dist, args, workload, world, rank, local, steps, war
         sums = [torch.zeros_like(mine) for _ in range(world)]
         dist.all_gather(sums, mine)
         for r in range(world):
-            lo_r, hi_r = ks.multigpu.shard_bounds(P_all, world, r) if strong else (0, P_all)
-            n_r = hi_r - lo_r
+            n_r = shard_len(r)
             got = (int(g_idx[r, :n_r].astype(np.int64).sum()), int((g_score[r, :n_r] & 0xFFFFFFFF).sum()))
             assert got == (int(sums[r][0].item()), int(sums[r][1].item())), f"rank {rank}: shard {r} of the gather is wrong"
             assert g_idx[r, :n_r].min() >= -1 and g_idx[r, :n_r].max() < N
@@ -545,6 +579,10 @@ def run_workload(ks, torch, dist, args, workload, world, rank, local, steps, war
     snap.close()
     del d_mask, flush
     torch.cuda.empty_cache()
+    if dumped is not None:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in dumped.items():
+            np.save(os.path.join(args.dump_outputs, f"{workload}_{name}.npy"), a)
     return res
 
 
@@ -574,10 +612,15 @@ def main():
     clocks = {}
 
     def stop_sampler():
+        nonlocal sampler
         if sampler:
             clocks.update(sampler.stop())
+            sampler = None
 
-    r = run_workload(ks, torch, dist, args, args.workload, world, rank, local, args.steps, args.warmup, stop_sampler)
+    try:
+        r = run_workload(ks, torch, dist, args, args.workload, world, rank, local, args.steps, args.warmup, stop_sampler)
+    finally:  # a failed run must not leave nvidia-smi running
+        stop_sampler()
     sec = None
     if world == 1 and args.workload == "c3" and not args.no_secondary:
         sec = run_workload(ks, torch, dist, args, "c2", 1, 0, local, args.steps, args.warmup)

@@ -9,6 +9,7 @@ import json
 import os
 import subprocess
 import sys
+import tempfile
 import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
@@ -16,14 +17,14 @@ SHAPES = {"c2": (10_000, 100_000, 100_000), "c3": (50_000, 1_000_000, 500_000)} 
 
 
 def native(workload, device=-1):
+    """The executable is built in a temporary directory: the source tree may be read-only."""
     libdir = os.path.join(ROOT, "kube-scheduler-rs-reference_b200")
-    build = os.path.join(libdir, "csrc", "build")
-    os.makedirs(build, exist_ok=True)
-    exe = os.path.join(build, "pack_bench")
-    subprocess.run(["g++", "-O2", "-std=c++17", "-I" + os.path.join(ROOT, "include"), os.path.join(ROOT, "examples", "pack_bench.cpp"),
-                    "-L" + libdir, "-lksched", "-Wl,-rpath," + libdir, "-pthread", "-o", exe], check=True)
     n, p, b = SHAPES[workload]
-    out = subprocess.run([exe, str(n), str(p), str(b), str(device)], check=True, capture_output=True, text=True).stdout
+    with tempfile.TemporaryDirectory(prefix="ks_pack_bench_") as tmp:
+        exe = os.path.join(tmp, "pack_bench")
+        subprocess.run(["g++", "-O2", "-std=c++17", "-I" + os.path.join(ROOT, "include"), os.path.join(ROOT, "examples", "pack_bench.cpp"),
+                        "-L" + libdir, "-lksched", "-Wl,-rpath," + libdir, "-pthread", "-o", exe], check=True)
+        out = subprocess.run([exe, str(n), str(p), str(b), str(device)], check=True, capture_output=True, text=True).stdout
     return json.loads(out)
 
 
