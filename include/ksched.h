@@ -55,9 +55,10 @@ extern "C" {
 /* ks_select flags */
 #define KS_SELECT_AUTO 0u
 #define KS_SELECT_FORCE_DIRECT 1u  /* per-cell kernel (any policy) */
-#define KS_SELECT_FORCE_BITPAR 2u  /* bit-parallel kernel (KS_SCORE_LEFTOVER only) */
+#define KS_SELECT_FORCE_BITPAR 2u  /* bit-parallel kernel (any policy) */
 #define KS_SELECT_TIMING 4u        /* record CUDA events around each kernel; read with ks_last_timings */
-#define KS_SELECT_NO_GRAPH 8u      /* all-device calls are replayed from a cached CUDA graph; this disables it */
+#define KS_SELECT_NO_GRAPH 8u      /* repeated calls whose buffers are device or pinned host memory are replayed from a
+                                      cached CUDA graph; this disables it */
 
 /* value limits enforced on inputs so that scores and sums stay inside int64 */
 #define KS_MAX_CPU_MILLI ((int64_t)1 << 36)

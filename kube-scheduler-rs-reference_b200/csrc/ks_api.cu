@@ -10,6 +10,7 @@
 #include <mutex>
 #include <thread>
 #include <algorithm>
+#include <type_traits>
 #include <vector>
 
 #include "ks_bitpar.h"
@@ -66,6 +67,71 @@ struct DevBuf {
     }
 };
 
+enum SelectPath : uint32_t { PATH_EMPTY, PATH_DIRECT, PATH_BITPAR };
+
+// Everything the launch sequence of a ks_select call depends on once it is captured into a CUDA graph.  The key has no
+// padding, so two keys are equal exactly when memcmp says so.
+struct SelectKey {
+    uint64_t P;
+    const void *req_cpu, *req_mem, *sel;
+    const void *node_idx, *score, *feasible_cnt, *mask;
+    uint64_t mask_row_bytes;
+    int32_t policy, pods_space, out_space, mask_space;
+    uint32_t flags, path;
+    cudaStream_t stream;
+    const void* ready_event;
+    uint64_t version;      // ks_snapshot::version
+    uint64_t devbuf_epoch; // g_devbuf_epoch
+    uint64_t bitpar_epoch; // BitparIndex::epoch
+    // the exchange descriptor, all zero without one: the captured kernels hold every peer pointer
+    uint64_t world, rank, n_peers;
+    const void *peer_node_idx[KS_MAX_PEERS], *peer_score[KS_MAX_PEERS], *peer_flag[KS_MAX_PEERS];
+    const void *local_flags, *local_state;
+};
+static_assert(std::has_unique_object_representations_v<SelectKey>, "SelectKey is compared with memcmp: no padding");
+
+// The launch sequence of the last ks_select that qualified, captured once and replayed while its key repeats.
+struct GraphCache {
+    cudaGraphExec_t exec = nullptr;
+    SelectKey key{};
+    bool valid = false;
+    uint64_t launches = 0; // kernels inside the cached graph
+
+    bool hit(const SelectKey& k) const { return valid && memcmp(&k, &key, sizeof(k)) == 0; }
+    void reset() {
+        if (exec) cudaGraphExecDestroy(exec);
+        exec = nullptr;
+        valid = false;
+    }
+    // enqueue() puts the launch sequence on `st` and returns KS_OK or an error code; on a key miss it is captured
+    template <class F>
+    int run(const SelectKey& k, cudaStream_t st, F&& enqueue) {
+        if (!hit(k)) {
+            reset();
+            CU_TRY(cudaStreamBeginCapture(st, cudaStreamCaptureModeThreadLocal));
+            const uint64_t launches_before = g_launches.load();
+            const int rc = enqueue();
+            launches = g_launches.load() - launches_before; // captured, not executed yet
+            g_launches -= launches;
+            cudaGraph_t graph = nullptr;
+            cudaError_t e = cudaStreamEndCapture(st, &graph);
+            if (rc) {
+                if (graph) cudaGraphDestroy(graph);
+                return rc;
+            }
+            if (e != cudaSuccess) return fail(KS_ERR_CUDA, "stream capture failed: %s", cudaGetErrorString(e));
+            e = cudaGraphInstantiate(&exec, graph, 0);
+            cudaGraphDestroy(graph);
+            if (e != cudaSuccess) return fail(KS_ERR_CUDA, "graph instantiate failed: %s", cudaGetErrorString(e));
+            key = k;
+            valid = true;
+        }
+        CU_TRY(cudaGraphLaunch(exec, st));
+        g_launches += launches;
+        return KS_OK;
+    }
+};
+
 struct ks_snapshot {
     int device = 0;
     cudaStream_t stream = nullptr;
@@ -77,18 +143,14 @@ struct ks_snapshot {
     void* h_stream = nullptr;                 // pinned staging of one streaming micro-batch (inputs and results)
     int sms = 0, coop = 0;
     cudaEvent_t ev[4] = {nullptr, nullptr, nullptr, nullptr};
-    // host-space calls are pipelined in pod chunks: chunk c+1 is copied in on copy_stream while chunk c computes
+    // large host-space calls are pipelined in two pod chunks: chunk 1 is copied in on copy_stream while chunk 0 computes
     cudaStream_t copy_stream = nullptr;
-    cudaEvent_t ev_cfork = nullptr, ev_in[4] = {nullptr, nullptr, nullptr, nullptr};
+    cudaEvent_t ev_cfork = nullptr, ev_in[2] = {nullptr, nullptr};
     bool timing_valid = false;
     bool derived_dirty = true; // prio + bit-parallel index must be rebuilt before the next select
     const char* last_path = "none";
     BitparIndex bp;
-    // CUDA-graph replay of the launch sequence of an all-device ks_select (same arguments, same snapshot state)
-    cudaGraphExec_t graph_exec = nullptr;
-    uint64_t graph_key[16] = {0};
-    bool graph_valid = false;
-    uint64_t graph_launches = 0; // kernels inside the cached graph
+    GraphCache graph;
     uint64_t version = 1; // bumped whenever device-side snapshot state or buffers change
     std::mutex mu;
 };
@@ -159,7 +221,7 @@ int ks_snapshot_create(int device, ks_snapshot** out) {
     for (int i = 0; i < 4 && e == cudaSuccess; i++) e = cudaEventCreate(&s->ev[i]);
     if (e == cudaSuccess) e = cudaStreamCreateWithFlags(&s->copy_stream, cudaStreamNonBlocking);
     if (e == cudaSuccess) e = cudaEventCreateWithFlags(&s->ev_cfork, cudaEventDisableTiming);
-    for (int i = 0; i < 4 && e == cudaSuccess; i++) e = cudaEventCreateWithFlags(&s->ev_in[i], cudaEventDisableTiming);
+    for (int i = 0; i < 2 && e == cudaSuccess; i++) e = cudaEventCreateWithFlags(&s->ev_in[i], cudaEventDisableTiming);
     if (e == cudaSuccess) e = s->flag.ensure(sizeof(int));
     if (e == cudaSuccess) e = s->xflag.ensure(sizeof(int));
     if (e == cudaSuccess) e = cudaMemset(s->xflag.p, 0, sizeof(int));
@@ -183,10 +245,10 @@ void ks_snapshot_destroy(ks_snapshot* s) {
     if (s->h_stream) cudaFreeHost(s->h_stream);
     for (DevBuf* b : bufs) b->release();
     bitpar_release(s->bp);
-    if (s->graph_exec) cudaGraphExecDestroy(s->graph_exec);
+    s->graph.reset();
     for (int i = 0; i < 4; i++)
         if (s->ev[i]) cudaEventDestroy(s->ev[i]);
-    for (int i = 0; i < 4; i++)
+    for (int i = 0; i < 2; i++)
         if (s->ev_in[i]) cudaEventDestroy(s->ev_in[i]);
     if (s->ev_cfork) cudaEventDestroy(s->ev_cfork);
     if (s->copy_stream) cudaStreamDestroy(s->copy_stream);
@@ -333,12 +395,12 @@ static int refresh_derived(ks_snapshot* s, cudaStream_t st) {
     return KS_OK;
 }
 
-static int copy_pods_in(ks_snapshot* s, const ks_pods* pods, cudaStream_t st) {
-    if (pods->mem_space == KS_MEM_DEVICE) return KS_OK;
-    const uint64_t P = pods->n;
-    CU_TRY(cudaMemcpyAsync(s->st_rc.p, pods->req_cpu, P * 8, cudaMemcpyHostToDevice, st));
-    CU_TRY(cudaMemcpyAsync(s->st_rm.p, pods->req_mem, P * 8, cudaMemcpyHostToDevice, st));
-    CU_TRY(cudaMemcpyAsync(s->st_sel.p, pods->sel, P * 8 * s->W, cudaMemcpyHostToDevice, st));
+// host-space pods [c0, c1) into the staging buffers that stage_pods prepared
+static int copy_pods_in(ks_snapshot* s, const ks_pods* pods, uint64_t c0, uint64_t c1, cudaStream_t st) {
+    const uint64_t m = c1 - c0, W = s->W;
+    CU_TRY(cudaMemcpyAsync(s->st_rc.as<int64_t>() + c0, pods->req_cpu + c0, m * 8, cudaMemcpyHostToDevice, st));
+    CU_TRY(cudaMemcpyAsync(s->st_rm.as<int64_t>() + c0, pods->req_mem + c0, m * 8, cudaMemcpyHostToDevice, st));
+    CU_TRY(cudaMemcpyAsync(s->st_sel.as<uint64_t>() + c0 * W, pods->sel + c0 * W, m * 8 * W, cudaMemcpyHostToDevice, st));
     return KS_OK;
 }
 
@@ -369,7 +431,7 @@ static int stage_pods(ks_snapshot* s, const ks_pods* pods, cudaStream_t st, PodV
     pv->req_mem = s->st_rm.as<int64_t>();
     pv->sel = s->st_sel.as<uint64_t>();
     if (st == nullptr) return KS_OK; // prepare only: the caller enqueues the copies itself (copy_pods_in)
-    return copy_pods_in(s, pods, st);
+    return copy_pods_in(s, pods, 0, P, st);
 }
 
 static int check_pods(const ks_snapshot* s, const ks_pods* pods) {
@@ -423,13 +485,12 @@ int ks_check_cell(ks_snapshot* s, int64_t req_cpu, int64_t req_mem, const uint64
     return (int)code;
 }
 
-int ks_select(ks_snapshot* s, const ks_pods* pods, int policy, uint32_t flags, ks_bindings* out, void* cuda_stream) {
+static int check_select_args(const ks_snapshot* s, const ks_pods* pods, int policy, uint32_t flags, const ks_bindings* out) {
     int rc = check_pods(s, pods);
     if (rc) return rc;
     if (!out) return fail(KS_ERR_INVALID, "out is NULL");
     if (policy != KS_SCORE_LEFTOVER && policy != KS_SCORE_LEAST_ALLOCATED) return fail(KS_ERR_INVALID, "bad policy");
     if ((flags & KS_SELECT_FORCE_BITPAR) && (flags & KS_SELECT_FORCE_DIRECT)) return fail(KS_ERR_INVALID, "bad flags");
-    const uint64_t P = pods->n;
     if (out->mask) {
         if (out->mask_row_bytes % 32 != 0 || out->mask_row_bytes < ks_mask_row_bytes(s->N))
             return fail(KS_ERR_INVALID, "mask_row_bytes must be a multiple of 32 and >= %llu",
@@ -448,49 +509,60 @@ int ks_select(ks_snapshot* s, const ks_pods* pods, int policy, uint32_t flags, k
             if (!xc->peer_node_idx[k] || !xc->peer_score[k] || !xc->peer_flag[k])
                 return fail(KS_ERR_INVALID, "exchange: NULL peer pointer %u", k);
     }
-    if (P == 0 && !xc) return KS_OK;
-    std::lock_guard<std::mutex> lk(s->mu);
-    CU_TRY(cudaSetDevice(s->device));
-    cudaStream_t st = cuda_stream ? (cudaStream_t)cuda_stream : s->stream;
-    const bool timing = (flags & KS_SELECT_TIMING) != 0;
-    PeerOut po;
-    if (xc) {
-        po.n = xc->n_peers;
-        po.world = xc->world;
-        po.rank = xc->rank;
-        for (uint32_t k = 0; k < xc->n_peers; k++) {
-            po.idx[k] = xc->peer_node_idx[k];
-            po.score[k] = xc->peer_score[k];
-            po.flag[k] = xc->peer_flag[k];
-        }
-        po.local_flags = xc->local_flags;
-        po.state = xc->local_state;
-    }
-    if (P == 0) { // an empty shard still takes part in the exchange: publish the sequence number, wait for the others
-        CU_TRY(launch_exchange_push(po, nullptr, nullptr, 0, st));
-        CU_TRY(launch_exchange_wait(po, s->xflag.as<int>(), st));
-        return KS_OK;
-    }
-    s->timing_valid = false;
-    if (timing) CU_TRY(cudaEventRecord(s->ev[0], st));
+    return KS_OK;
+}
 
+static PeerOut peer_out(const ks_exchange* xc) {
+    PeerOut po;
+    if (!xc) return po;
+    po.n = xc->n_peers;
+    po.world = xc->world;
+    po.rank = xc->rank;
+    for (uint32_t k = 0; k < xc->n_peers; k++) {
+        po.idx[k] = xc->peer_node_idx[k];
+        po.score[k] = xc->peer_score[k];
+        po.flag[k] = xc->peer_flag[k];
+    }
+    po.local_flags = xc->local_flags;
+    po.state = xc->local_state;
+    return po;
+}
+
+struct SelectPlan {
+    SelectPath path;
+    SelectLaunch L;                        // the whole call; host-space outputs point to their device staging
+    PartialView part;                      // direct path: partial results per node chunk
+    uint32_t node_chunks, tiles_per_chunk; // direct path: split of the node dimension across CTAs
+    uint32_t pod_chunks;                   // 2 = the host-space pipeline, else 1
+};
+
+// Picks the path and the pod chunking and makes every allocation of the call: the launch sequence that follows may be
+// stream-captured, and nothing may allocate inside a capture.
+static int plan_select(ks_snapshot* s, const ks_pods* pods, int policy, uint32_t flags, const ks_bindings* out,
+                       const PeerOut& po, cudaStream_t st, SelectPlan* pl) {
+    const uint64_t P = pods->n;
     // the per-cell kernel needs no derived state; the bit-parallel index is (re)built lazily
     const bool may_bitpar = (flags & KS_SELECT_FORCE_BITPAR) ||
-                            (!(flags & KS_SELECT_FORCE_DIRECT) && (uint64_t)P * s->N >= (1ull << 24));
+                            (!(flags & KS_SELECT_FORCE_DIRECT) && P * s->N >= (1ull << 24));
     if (may_bitpar) {
-        rc = refresh_derived(s, st);
+        const int rc = refresh_derived(s, st);
         if (rc) return rc;
     }
-
-    const bool out_host = out->mem_space == KS_MEM_HOST;
-    const bool mask_host = out->mask && out->mask_space == KS_MEM_HOST;
-    OutView ov;
+    SelectLaunch& L = pl->L;
+    L.nt = node_table(s);
+    L.pv.P = (uint32_t)P;
+    L.policy = policy;
+    L.stream = st;
+    L.po = po;
+    OutView& ov = L.ov;
     ov.node_idx = out->node_idx;
     ov.score = out->score;
     ov.cnt = out->feasible_cnt;
     ov.mask = reinterpret_cast<uint32_t*>(out->mask);
     ov.mask_row_words = out->mask_row_bytes / 4;
     ov.mask_valid_words = (uint32_t)(ks_mask_row_bytes(s->N) / 4);
+    const bool out_host = out->mem_space == KS_MEM_HOST;
+    const bool mask_host = out->mask && out->mask_space == KS_MEM_HOST;
     if (out_host) {
         if (out->node_idx) {
             CU_TRY(s->st_idx.ensure(P * 4));
@@ -509,193 +581,218 @@ int ks_select(ks_snapshot* s, const ks_pods* pods, int policy, uint32_t flags, k
         CU_TRY(s->st_mask.ensure(P * out->mask_row_bytes));
         ov.mask = s->st_mask.as<uint32_t>();
     }
-
-    if (s->N == 0) { // empty node store: every pod gets None (src/main.rs:56,70)
-        if (ov.node_idx) CU_TRY(cudaMemsetAsync(ov.node_idx, 0xff, P * 4, st));
-        if (ov.score) CU_TRY(cudaMemsetAsync(ov.score, 0, P * 8, st));
-        if (ov.cnt) CU_TRY(cudaMemsetAsync(ov.cnt, 0, P * 4, st));
-        if (xc) {
-            CU_TRY(launch_exchange_push(po, ov.node_idx, ov.score, (uint32_t)P, st));
-            CU_TRY(launch_exchange_wait(po, s->xflag.as<int>(), st));
-        }
-        if (out_host) {
-            if (out->node_idx) CU_TRY(cudaMemcpyAsync(out->node_idx, ov.node_idx, P * 4, cudaMemcpyDeviceToHost, st));
-            if (out->score) CU_TRY(cudaMemcpyAsync(out->score, ov.score, P * 8, cudaMemcpyDeviceToHost, st));
-            if (out->feasible_cnt) CU_TRY(cudaMemcpyAsync(out->feasible_cnt, ov.cnt, P * 4, cudaMemcpyDeviceToHost, st));
-        }
+    pl->pod_chunks = 1;
+    if (s->N == 0) {
+        pl->path = PATH_EMPTY;
         s->last_path = "empty";
+        return KS_OK;
+    }
+    int rc = stage_pods(s, pods, nullptr, &L.pv);
+    if (rc) return rc;
+    bool use_bitpar = false;
+    if (flags & KS_SELECT_FORCE_BITPAR) use_bitpar = true;
+    else if (!(flags & KS_SELECT_FORCE_DIRECT))
+        use_bitpar = may_bitpar && bitpar_profitable(s->bp, L.pv.P);
+    if (use_bitpar) {
+        cudaError_t e = bitpar_prepare(s->bp, L.pv.P);
+        if (e != cudaSuccess) return fail(KS_ERR_CUDA, "bit-parallel prepare failed: %s", cudaGetErrorString(e));
     } else {
-        SelectLaunch L;
-        L.nt = node_table(s);
-        rc = stage_pods(s, pods, nullptr, &L.pv); // prepare; copies are part of the (possibly captured) sequence
-        if (rc) return rc;
-        L.ov = ov;
-        L.policy = policy;
-        L.stream = st;
-        L.po = po;
-        bool use_bitpar = false;
-        if (flags & KS_SELECT_FORCE_BITPAR) use_bitpar = true;
-        else if (!(flags & KS_SELECT_FORCE_DIRECT))
-            use_bitpar = may_bitpar && bitpar_profitable(s->bp, L.pv.P);
-        // everything that allocates happens before the (possibly captured) launch sequence
-        uint32_t n_chunks = 1, tiles_per_chunk = 0;
-        PartialView part{nullptr, nullptr, nullptr};
-        if (use_bitpar) {
-            cudaError_t e = bitpar_prepare(s->bp, L.pv.P);
-            if (e != cudaSuccess) return fail(KS_ERR_CUDA, "bit-parallel prepare failed: %s", cudaGetErrorString(e));
-        } else {
-            const uint32_t n_tiles = s->Npad / TILE_N;
-            const uint32_t pod_ctas = (L.pv.P + direct_pods_per_cta(s->W) - 1) / direct_pods_per_cta(s->W);
-            const uint32_t want_ctas = 2u * (uint32_t)s->sms; // at least two CTAs per SM
-            if (pod_ctas < want_ctas) n_chunks = std::min<uint32_t>(n_tiles, (want_ctas + pod_ctas - 1) / pod_ctas);
-            tiles_per_chunk = (n_tiles + n_chunks - 1) / n_chunks;
-            n_chunks = (n_tiles + tiles_per_chunk - 1) / tiles_per_chunk;
-            if (n_chunks > 1) {
-                CU_TRY(s->part_key.ensure((size_t)n_chunks * P * 8));
-                CU_TRY(s->part_idx.ensure((size_t)n_chunks * P * 4));
-                CU_TRY(s->part_cnt.ensure((size_t)n_chunks * P * 4));
-                part.key = s->part_key.as<int64_t>();
-                part.idx = s->part_idx.as<int32_t>();
-                part.cnt = s->part_cnt.as<uint32_t>();
-            }
-            cudaError_t e = prepare_select_direct(s->W);
-            if (e != cudaSuccess) return fail(KS_ERR_CUDA, "direct prepare failed: %s", cudaGetErrorString(e));
+        const uint32_t n_tiles = s->Npad / TILE_N;
+        const uint32_t pod_ctas = (L.pv.P + direct_pods_per_cta(s->W) - 1) / direct_pods_per_cta(s->W);
+        const uint32_t want_ctas = 2u * (uint32_t)s->sms; // at least two CTAs per SM
+        uint32_t n_chunks = 1;
+        if (pod_ctas < want_ctas) n_chunks = std::min<uint32_t>(n_tiles, (want_ctas + pod_ctas - 1) / pod_ctas);
+        pl->tiles_per_chunk = (n_tiles + n_chunks - 1) / n_chunks;
+        pl->node_chunks = (n_tiles + pl->tiles_per_chunk - 1) / pl->tiles_per_chunk;
+        if (pl->node_chunks > 1) {
+            CU_TRY(s->part_key.ensure((size_t)pl->node_chunks * P * 8));
+            CU_TRY(s->part_idx.ensure((size_t)pl->node_chunks * P * 4));
+            CU_TRY(s->part_cnt.ensure((size_t)pl->node_chunks * P * 4));
+            pl->part.key = s->part_key.as<int64_t>();
+            pl->part.idx = s->part_idx.as<int32_t>();
+            pl->part.cnt = s->part_cnt.as<uint32_t>();
         }
-        s->last_path = use_bitpar ? "bitpar" : "direct";
-        // Host-space batches on the bit-parallel path are pipelined in two pod chunks: the second chunk is copied in
-        // on copy_stream while the first computes, and the bindings of a chunk travel back under the next chunk's
-        // mask kernel.  (Each chunk is an independent select over its pod range; scratch is reused because a chunk
-        // starts only after the previous chunk's auxiliary-stream work has joined.)
-        const uint32_t n_pipe = (use_bitpar && pods->mem_space == KS_MEM_HOST && out_host && !mask_host && !timing &&
-                                 P >= 262144) // below that the per-chunk launch overhead outweighs the overlap (measured at 100k pods)
-                                    ? 2u
-                                    : 1u;
-        auto enqueue = [&]() -> int {
-            if (n_pipe == 1) {
-                int crc = copy_pods_in(s, pods, st);
-                if (crc) return crc;
-            } else {
-                CU_TRY(cudaEventRecord(s->ev_cfork, st));
-                CU_TRY(cudaStreamWaitEvent(s->copy_stream, s->ev_cfork, 0));
-                for (uint32_t c = 0; c < n_pipe; c++) {
-                    const uint64_t c0 = P * c / n_pipe, c1 = P * (c + 1) / n_pipe, m = c1 - c0;
-                    CU_TRY(cudaMemcpyAsync(s->st_rc.as<int64_t>() + c0, pods->req_cpu + c0, m * 8, cudaMemcpyHostToDevice,
-                                           s->copy_stream));
-                    CU_TRY(cudaMemcpyAsync(s->st_rm.as<int64_t>() + c0, pods->req_mem + c0, m * 8, cudaMemcpyHostToDevice,
-                                           s->copy_stream));
-                    CU_TRY(cudaMemcpyAsync(s->st_sel.as<uint64_t>() + c0 * s->W, pods->sel + c0 * s->W, m * 8 * s->W,
-                                           cudaMemcpyHostToDevice, s->copy_stream));
-                    CU_TRY(cudaEventRecord(s->ev_in[c], s->copy_stream));
-                }
-                for (uint32_t c = 0; c < n_pipe; c++) {
-                    const uint64_t c0 = P * c / n_pipe, c1 = P * (c + 1) / n_pipe, m = c1 - c0;
-                    CU_TRY(cudaStreamWaitEvent(st, s->ev_in[c], 0));
-                    SelectLaunch Lc = L;
-                    Lc.pv.req_cpu += c0;
-                    Lc.pv.req_mem += c0;
-                    Lc.pv.sel += c0 * s->W;
-                    Lc.pv.P = (uint32_t)m;
-                    if (Lc.ov.node_idx) Lc.ov.node_idx += c0;
-                    if (Lc.ov.score) Lc.ov.score += c0;
-                    if (Lc.ov.cnt) Lc.ov.cnt += c0;
-                    if (Lc.ov.mask) Lc.ov.mask += c0 * Lc.ov.mask_row_words;
-                    Lc.host_node_idx = out->node_idx ? out->node_idx + c0 : nullptr;
-                    Lc.host_score = out->score ? out->score + c0 : nullptr;
-                    cudaError_t e = bitpar_select(s->bp, Lc, nullptr, nullptr);
-                    if (e != cudaSuccess) return fail(KS_ERR_CUDA, "bit-parallel select failed: %s", cudaGetErrorString(e));
-                    if (Lc.host_node_idx)
-                        CU_TRY(cudaMemcpyAsync(Lc.host_node_idx, Lc.ov.node_idx, m * 4, cudaMemcpyDeviceToHost, st));
-                    if (Lc.host_score) CU_TRY(cudaMemcpyAsync(Lc.host_score, Lc.ov.score, m * 8, cudaMemcpyDeviceToHost, st));
-                    if (out->feasible_cnt)
-                        CU_TRY(cudaMemcpyAsync(out->feasible_cnt + c0, Lc.ov.cnt, m * 4, cudaMemcpyDeviceToHost, st));
-                }
-                return KS_OK;
-            }
-            L.host_node_idx = out_host ? out->node_idx : nullptr; // served early by the launcher when it can
-            L.host_score = out_host ? out->score : nullptr;
-            L.ready_event = out_host ? nullptr : (cudaEvent_t)out->bindings_ready_event;
-            if (use_bitpar) {
-                cudaError_t e = bitpar_select(s->bp, L, timing ? s->ev[1] : nullptr, timing ? s->ev[2] : nullptr);
-                if (e != cudaSuccess) return fail(KS_ERR_CUDA, "bit-parallel select failed: %s", cudaGetErrorString(e));
-            } else {
-                if (timing) CU_TRY(cudaEventRecord(s->ev[1], st));
-                cudaError_t e = launch_select_direct(L, part, n_chunks, tiles_per_chunk);
-                if (e != cudaSuccess) return fail(KS_ERR_CUDA, "direct select failed: %s", cudaGetErrorString(e));
-                if (timing) CU_TRY(cudaEventRecord(s->ev[2], st));
-                if (xc) CU_TRY(launch_exchange_push(po, ov.node_idx, ov.score, (uint32_t)P, st));
-            }
-            // fused all-gather: this rank's bindings went out from the argmax kernels (bit-parallel path) or the push
-            // kernel; the call's stream work ends when every other rank's bindings have arrived here
-            if (xc) CU_TRY(launch_exchange_wait(po, s->xflag.as<int>(), st));
-            if (out_host) {
-                if (L.host_node_idx) CU_TRY(cudaMemcpyAsync(out->node_idx, ov.node_idx, P * 4, cudaMemcpyDeviceToHost, st));
-                if (L.host_score) CU_TRY(cudaMemcpyAsync(out->score, ov.score, P * 8, cudaMemcpyDeviceToHost, st));
-                if (out->feasible_cnt)
-                    CU_TRY(cudaMemcpyAsync(out->feasible_cnt, ov.cnt, P * 4, cudaMemcpyDeviceToHost, st));
-            }
-            if (mask_host)
-                CU_TRY(cudaMemcpyAsync(out->mask, ov.mask, P * out->mask_row_bytes, cudaMemcpyDeviceToHost, st));
-            if (L.ready_event) { // not served earlier (per-cell path): the bindings are final here
-                cudaStreamCaptureStatus cs = cudaStreamCaptureStatusNone;
-                CU_TRY(cudaStreamIsCapturing(st, &cs));
-                CU_TRY(cudaEventRecordWithFlags(L.ready_event, st, cs == cudaStreamCaptureStatusActive ? cudaEventRecordExternal
-                                                                                                   : cudaEventRecordDefault));
-            }
-            return KS_OK;
-        };
-        // Replay from a cached CUDA graph when the call repeats (same buffers, same snapshot state).  Host buffers
-        // qualify only if they are pinned (a captured copy from pageable memory is not allowed).
-        const uint64_t key[16] = {P, (uint64_t)pods->req_cpu, (uint64_t)pods->req_mem, (uint64_t)pods->sel,
-                                  (uint64_t)out->node_idx, (uint64_t)out->score, (uint64_t)out->feasible_cnt,
-                                  (uint64_t)out->mask, out->mask_row_bytes,
-                                  (uint64_t)policy | ((uint64_t)pods->mem_space << 8) | ((uint64_t)out->mem_space << 9) |
-                                      ((uint64_t)out->mask_space << 10),
-                                  (uint64_t)flags ^ ((uint64_t)out->bindings_ready_event << 8) ^ ((uint64_t)(xc ? xc->local_state : nullptr) << 20), (uint64_t)st, s->version, (uint64_t)use_bitpar,
-                                  g_devbuf_epoch.load(), s->bp.epoch};
-        const bool key_hit = s->graph_valid && memcmp(key, s->graph_key, sizeof(key)) == 0;
-        bool graph_ok = !timing && !(flags & KS_SELECT_NO_GRAPH);
-        if (graph_ok && !key_hit) {
-            if (pods->mem_space == KS_MEM_HOST)
-                graph_ok = is_pinned_host(pods->req_cpu) && is_pinned_host(pods->req_mem) && is_pinned_host(pods->sel);
-            if (graph_ok && out_host)
-                graph_ok = is_pinned_host(out->node_idx) && is_pinned_host(out->score) && is_pinned_host(out->feasible_cnt);
-            if (graph_ok && mask_host) graph_ok = is_pinned_host(out->mask);
+        cudaError_t e = prepare_select_direct(s->W);
+        if (e != cudaSuccess) return fail(KS_ERR_CUDA, "direct prepare failed: %s", cudaGetErrorString(e));
+    }
+    pl->path = use_bitpar ? PATH_BITPAR : PATH_DIRECT;
+    s->last_path = use_bitpar ? "bitpar" : "direct";
+    // Host-space batches on the bit-parallel path are pipelined in two pod chunks: the second chunk is copied in on
+    // copy_stream while the first computes, and the bindings of a chunk travel back under the next chunk's mask kernel.
+    // (Each chunk is an independent select over its pod range; scratch is reused because a chunk starts only after the
+    // previous chunk's auxiliary-stream work has joined.)
+    if (use_bitpar && pods->mem_space == KS_MEM_HOST && out_host && !mask_host && !(flags & KS_SELECT_TIMING) &&
+        P >= 262144) // below that the per-chunk launch overhead outweighs the overlap (measured at 100k pods)
+        pl->pod_chunks = 2;
+    return KS_OK;
+}
+
+// One pod chunk of the planned path.  Clears what it served of Lc.host_node_idx / host_score / ready_event.
+static int launch_chunk(ks_snapshot* s, const SelectPlan& pl, SelectLaunch& Lc, bool timing) {
+    const cudaStream_t st = Lc.stream;
+    const uint64_t m = Lc.pv.P;
+    cudaError_t e = cudaSuccess;
+    switch (pl.path) {
+        case PATH_EMPTY: // every pod gets None (src/main.rs:56,70)
+            if (Lc.ov.node_idx) CU_TRY(cudaMemsetAsync(Lc.ov.node_idx, 0xff, m * 4, st));
+            if (Lc.ov.score) CU_TRY(cudaMemsetAsync(Lc.ov.score, 0, m * 8, st));
+            if (Lc.ov.cnt) CU_TRY(cudaMemsetAsync(Lc.ov.cnt, 0, m * 4, st));
+            CU_TRY(launch_exchange_push(Lc.po, Lc.ov.node_idx, Lc.ov.score, (uint32_t)m, st));
+            break;
+        case PATH_DIRECT:
+            if (timing) CU_TRY(cudaEventRecord(s->ev[1], st));
+            e = launch_select_direct(Lc, pl.part, pl.node_chunks, pl.tiles_per_chunk);
+            if (e != cudaSuccess) return fail(KS_ERR_CUDA, "direct select failed: %s", cudaGetErrorString(e));
+            if (timing) CU_TRY(cudaEventRecord(s->ev[2], st));
+            CU_TRY(launch_exchange_push(Lc.po, Lc.ov.node_idx, Lc.ov.score, (uint32_t)m, st));
+            break;
+        case PATH_BITPAR: // the argmax kernels send the bindings to the peers themselves
+            e = bitpar_select(s->bp, Lc, timing ? s->ev[1] : nullptr, timing ? s->ev[2] : nullptr);
+            if (e != cudaSuccess) return fail(KS_ERR_CUDA, "bit-parallel select failed: %s", cudaGetErrorString(e));
+            break;
+    }
+    return KS_OK;
+}
+
+// The launch sequence of a planned ks_select: per pod chunk, wait for its input copy, launch it, copy back the host
+// outputs the launcher has not served; then the per-call tail.  Allocates nothing.
+static int enqueue_select(ks_snapshot* s, const ks_pods* pods, const ks_bindings* out, const SelectPlan& pl, bool timing) {
+    const SelectLaunch& L = pl.L;
+    const cudaStream_t st = L.stream;
+    const uint64_t P = L.pv.P, W = s->W;
+    const uint32_t n = pl.pod_chunks;
+    const bool out_host = out->mem_space == KS_MEM_HOST;
+    if (pl.path != PATH_EMPTY && pods->mem_space == KS_MEM_HOST) {
+        const cudaStream_t cs = n > 1 ? s->copy_stream : st;
+        if (n > 1) {
+            CU_TRY(cudaEventRecord(s->ev_cfork, st));
+            CU_TRY(cudaStreamWaitEvent(cs, s->ev_cfork, 0));
         }
-        if (graph_ok) {
-            if (!key_hit) {
-                if (s->graph_exec) cudaGraphExecDestroy(s->graph_exec);
-                s->graph_exec = nullptr;
-                s->graph_valid = false;
-                CU_TRY(cudaStreamBeginCapture(st, cudaStreamCaptureModeThreadLocal));
-                const uint64_t launches_before = g_launches.load();
-                const int erc = enqueue();
-                s->graph_launches = g_launches.load() - launches_before; // captured, not executed yet
-                g_launches -= s->graph_launches;
-                cudaGraph_t graph = nullptr;
-                cudaError_t e = cudaStreamEndCapture(st, &graph);
-                if (erc) {
-                    if (graph) cudaGraphDestroy(graph);
-                    return erc;
-                }
-                if (e != cudaSuccess) return fail(KS_ERR_CUDA, "stream capture failed: %s", cudaGetErrorString(e));
-                e = cudaGraphInstantiate(&s->graph_exec, graph, 0);
-                cudaGraphDestroy(graph);
-                if (e != cudaSuccess) return fail(KS_ERR_CUDA, "graph instantiate failed: %s", cudaGetErrorString(e));
-                memcpy(s->graph_key, key, sizeof(key));
-                s->graph_valid = true;
-            }
-            CU_TRY(cudaGraphLaunch(s->graph_exec, st));
-            g_launches += s->graph_launches;
-        } else {
-            rc = enqueue();
+        for (uint32_t c = 0; c < n; c++) {
+            const int rc = copy_pods_in(s, pods, P * c / n, P * (c + 1) / n, cs);
             if (rc) return rc;
+            if (n > 1) CU_TRY(cudaEventRecord(s->ev_in[c], cs));
         }
     }
+    cudaEvent_t ready = out_host ? nullptr : (cudaEvent_t)out->bindings_ready_event;
+    for (uint32_t c = 0; c < n; c++) {
+        const uint64_t c0 = P * c / n, m = P * (c + 1) / n - c0;
+        if (n > 1) CU_TRY(cudaStreamWaitEvent(st, s->ev_in[c], 0));
+        SelectLaunch Lc = L;
+        Lc.pv.req_cpu += c0;
+        Lc.pv.req_mem += c0;
+        Lc.pv.sel += c0 * W;
+        Lc.pv.P = (uint32_t)m;
+        if (Lc.ov.node_idx) Lc.ov.node_idx += c0;
+        if (Lc.ov.score) Lc.ov.score += c0;
+        if (Lc.ov.cnt) Lc.ov.cnt += c0;
+        if (Lc.ov.mask) Lc.ov.mask += c0 * Lc.ov.mask_row_words;
+        Lc.host_node_idx = out_host && out->node_idx ? out->node_idx + c0 : nullptr;
+        Lc.host_score = out_host && out->score ? out->score + c0 : nullptr;
+        Lc.ready_event = ready;
+        const int rc = launch_chunk(s, pl, Lc, timing);
+        if (rc) return rc;
+        ready = Lc.ready_event;
+        if (Lc.host_node_idx) CU_TRY(cudaMemcpyAsync(Lc.host_node_idx, Lc.ov.node_idx, m * 4, cudaMemcpyDeviceToHost, st));
+        if (Lc.host_score) CU_TRY(cudaMemcpyAsync(Lc.host_score, Lc.ov.score, m * 8, cudaMemcpyDeviceToHost, st));
+        if (out_host && out->feasible_cnt)
+            CU_TRY(cudaMemcpyAsync(out->feasible_cnt + c0, Lc.ov.cnt, m * 4, cudaMemcpyDeviceToHost, st));
+    }
+    // The per-call tail runs once, after the last chunk.  Two chunks need host-space outputs and no host-space mask, while
+    // an exchange and a ready event need device-space outputs: with two chunks the tail has nothing to do.
+    // With an exchange, the call's stream work ends when every other rank's bindings have arrived here.
+    CU_TRY(launch_exchange_wait(L.po, s->xflag.as<int>(), st));
+    if (out->mask && out->mask_space == KS_MEM_HOST && pl.path != PATH_EMPTY) // the empty store writes no mask
+        CU_TRY(cudaMemcpyAsync(out->mask, L.ov.mask, P * out->mask_row_bytes, cudaMemcpyDeviceToHost, st));
+    if (ready) CU_TRY(record_ready_event(ready, st)); // not served by the launcher: the bindings are final here
+    return KS_OK;
+}
+
+static SelectKey select_key(const ks_snapshot* s, const ks_pods* pods, int policy, uint32_t flags, const ks_bindings* out,
+                            cudaStream_t st, SelectPath path) {
+    SelectKey k{};
+    k.P = pods->n;
+    k.req_cpu = pods->req_cpu;
+    k.req_mem = pods->req_mem;
+    k.sel = pods->sel;
+    k.node_idx = out->node_idx;
+    k.score = out->score;
+    k.feasible_cnt = out->feasible_cnt;
+    k.mask = out->mask;
+    k.mask_row_bytes = out->mask_row_bytes;
+    k.policy = policy;
+    k.pods_space = pods->mem_space;
+    k.out_space = out->mem_space;
+    k.mask_space = out->mask_space;
+    k.flags = flags;
+    k.path = path;
+    k.stream = st;
+    k.ready_event = out->bindings_ready_event;
+    k.version = s->version;
+    k.devbuf_epoch = g_devbuf_epoch.load();
+    k.bitpar_epoch = s->bp.epoch;
+    if (const ks_exchange* xc = out->exchange) {
+        k.world = xc->world;
+        k.rank = xc->rank;
+        k.n_peers = xc->n_peers;
+        for (uint32_t i = 0; i < xc->n_peers; i++) {
+            k.peer_node_idx[i] = xc->peer_node_idx[i];
+            k.peer_score[i] = xc->peer_score[i];
+            k.peer_flag[i] = xc->peer_flag[i];
+        }
+        k.local_flags = xc->local_flags;
+        k.local_state = xc->local_state;
+    }
+    return k;
+}
+
+// a captured copy from pageable host memory is not allowed: a call with host-space buffers is replayed only if they are pinned
+static bool host_buffers_pinned(const ks_pods* pods, const ks_bindings* out) {
+    if (pods->mem_space == KS_MEM_HOST &&
+        !(is_pinned_host(pods->req_cpu) && is_pinned_host(pods->req_mem) && is_pinned_host(pods->sel)))
+        return false;
+    if (out->mem_space == KS_MEM_HOST &&
+        !(is_pinned_host(out->node_idx) && is_pinned_host(out->score) && is_pinned_host(out->feasible_cnt)))
+        return false;
+    return !(out->mask && out->mask_space == KS_MEM_HOST) || is_pinned_host(out->mask);
+}
+
+int ks_select(ks_snapshot* s, const ks_pods* pods, int policy, uint32_t flags, ks_bindings* out, void* cuda_stream) {
+    int rc = check_select_args(s, pods, policy, flags, out);
+    if (rc) return rc;
+    const uint64_t P = pods->n;
+    if (P == 0 && !out->exchange) return KS_OK;
+    std::lock_guard<std::mutex> lk(s->mu);
+    CU_TRY(cudaSetDevice(s->device));
+    cudaStream_t st = cuda_stream ? (cudaStream_t)cuda_stream : s->stream;
+    const bool timing = (flags & KS_SELECT_TIMING) != 0;
+    const PeerOut po = peer_out(out->exchange);
+    if (P == 0) { // an empty shard still takes part in the exchange: publish the sequence number, wait for the others
+        CU_TRY(launch_exchange_push(po, nullptr, nullptr, 0, st));
+        CU_TRY(launch_exchange_wait(po, s->xflag.as<int>(), st));
+        return KS_OK;
+    }
+    s->timing_valid = false;
+    if (timing) CU_TRY(cudaEventRecord(s->ev[0], st));
+    SelectPlan pl{};
+    rc = plan_select(s, pods, policy, flags, out, po, st, &pl);
+    if (rc) return rc;
+    auto enqueue = [&] { return enqueue_select(s, pods, out, pl, timing); };
+    // The kernel paths replay a repeated call from the cached CUDA graph; the pinned check only runs on a key miss.
+    const SelectKey key = select_key(s, pods, policy, flags, out, st, pl.path);
+    if (pl.path != PATH_EMPTY && !timing && !(flags & KS_SELECT_NO_GRAPH) &&
+        (s->graph.hit(key) || host_buffers_pinned(pods, out)))
+        rc = s->graph.run(key, st, enqueue);
+    else
+        rc = enqueue();
+    if (rc) return rc;
     if (timing) {
         CU_TRY(cudaEventRecord(s->ev[3], st));
         s->timing_valid = s->N != 0;
     }
-    if (out_host || mask_host || pods->mem_space == KS_MEM_HOST || timing) CU_TRY(cudaStreamSynchronize(st));
+    const bool mask_host = out->mask && out->mask_space == KS_MEM_HOST;
+    if (out->mem_space == KS_MEM_HOST || mask_host || pods->mem_space == KS_MEM_HOST || timing)
+        CU_TRY(cudaStreamSynchronize(st));
     return KS_OK;
 }
 
@@ -887,8 +984,7 @@ int ks_stream_bind(ks_snapshot* s, const ks_pods* pods, int policy, int32_t* out
     const uint64_t n = pods->n;
     const uint32_t W = s->W;
     if (policy != KS_SCORE_LEFTOVER && policy != KS_SCORE_LEAST_ALLOCATED) return fail(KS_ERR_INVALID, "bad policy");
-    static const bool host_loop = getenv("KS_STREAM_HOST_LOOP") != nullptr; // A/B switch: the round-1 host-driven loop
-    if (n > 0 && n <= STREAM_BATCH_MAX && s->N > 0 && s->coop && !host_loop) {
+    if (n > 0 && n <= STREAM_BATCH_MAX && s->N > 0 && s->coop) {
         // device-side loop: one H2D, ONE cooperative launch that runs every round, one D2H
         std::lock_guard<std::mutex> lk(s->mu);
         CU_TRY(cudaSetDevice(s->device));
@@ -946,7 +1042,7 @@ int ks_stream_bind(ks_snapshot* s, const ks_pods* pods, int policy, int32_t* out
         s->last_path = "stream_batch";
         return KS_OK;
     }
-    try { // host-driven loop (large batches, A/B): its vectors must not throw across the ABI
+    try { // host-driven loop (large batches, no cooperative launch): its vectors must not throw across the ABI
         std::vector<uint64_t> pending(n);
         for (uint64_t i = 0; i < n; i++) {
             pending[i] = i;

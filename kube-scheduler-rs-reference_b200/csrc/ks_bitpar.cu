@@ -1348,7 +1348,7 @@ cudaError_t bitpar_build(BitparIndex& ix, const NodeTable& nt, int64_t* prio, cu
                                                     stride, ix.ordL_s0, ix.ordL_idx);
     g_launches += 4;
     if ((e = cudaGetLastError()) != cudaSuccess) return e;
-    BitparLayout lay{}, layP{};
+    BitparLayout layP{};
     if (!make_layout_flat(nt.N, nt.W, &layP)) return cudaSuccess; // direct path only
     if (layP.blob_bytes > ix.cap_blobP) {
         const size_t cap = (size_t)layP.blob_bytes + layP.blob_bytes / 8;
@@ -1386,8 +1386,6 @@ cudaError_t bitpar_build(BitparIndex& ix, const NodeTable& nt, int64_t* prio, cu
         g_launches++;
         if ((e = cudaGetLastError()) != cudaSuccess) return e;
         ix.lay_r = lr;
-        lay.nt = RW_TILES; // bitpar_profitable: (pod, tile) items
-        lay.ncb = lr.ncb;
     }
     k_build_tile<<<layP.nt, 288, 0, st>>>(nt, ix.gposC, ix.gposM, ix.ord_idx, ix.blobP, layP);
     g_launches++;
@@ -1397,7 +1395,6 @@ cudaError_t bitpar_build(BitparIndex& ix, const NodeTable& nt, int64_t* prio, cu
     k_build_eval<<<(Nord + 255) / 256, 256, 0, st>>>(nt, ix.ordL_idx, Nord, ix.evalL, ix.hintL);
     g_launches += 2;
     if ((e = cudaGetLastError()) != cudaSuccess) return e;
-    ix.lay = lay;
     ix.layP = layP;
     ix.valid = true;
     ix.epoch = g_regrow_epoch.load();
@@ -1407,7 +1404,7 @@ cudaError_t bitpar_build(BitparIndex& ix, const NodeTable& nt, int64_t* prio, cu
 bool bitpar_profitable(const BitparIndex& ix, uint32_t P) {
     // below ~16M cells the per-call rank pass and blob staging outweigh the per-cell kernel;
     // the mask kernel indexes (pod, tile) items with 32 bits
-    return ix.valid && (uint64_t)P * ix.N >= (1ull << 24) && (uint64_t)P * ix.lay.nt < (1ull << 31);
+    return ix.valid && (uint64_t)P * ix.N >= (1ull << 24) && (uint64_t)P * RW_TILES < (1ull << 31);
 }
 
 template <int W, int THREADS>
@@ -1461,7 +1458,7 @@ template <int W>
 static cudaError_t select_w(BitparIndex& ix, SelectLaunch& L, cudaEvent_t before_mask, cudaEvent_t after_mask) {
     cudaError_t e;
     const uint32_t P = L.pv.P;
-    if ((uint64_t)P * ix.lay.nt >= (1ull << 31)) return cudaErrorInvalidValue;
+    if ((uint64_t)P * RW_TILES >= (1ull << 31)) return cudaErrorInvalidValue;
     if ((e = bitpar_prepare(ix, P)) != cudaSuccess) return e; // no-op when the caller prepared already
     const bool need_mask_pass = L.ov.mask || L.ov.cnt;
     const int sms = ix.sms;
@@ -1494,7 +1491,7 @@ static cudaError_t select_w(BitparIndex& ix, SelectLaunch& L, cudaEvent_t before
     const uint32_t warps = (uint32_t)threads / 32;
     const uint32_t mask_grid = (uint32_t)std::min<uint64_t>((uint64_t)mask_sms, (F + warps - 1) / warps);
     k_pod_ranks<<<rank_grid, RANK_THREADS, rank_smem, L.stream>>>(L.pv, ix.sortedC, ix.sortedM, ix.N, ix.splC, ix.splM, ix.n_spl, ix.spl_stride,
-                                                 ix.pod_ranks, (need_mask_pass && ix.lay.ncb > 1) ? L.ov.cnt : nullptr, ix.W,
+                                                 ix.pod_ranks, (need_mask_pass && ix.lay_r.ncb > 1) ? L.ov.cnt : nullptr, ix.W,
                                                  need_mask_pass ? ix.rec_s : nullptr, ix.cursor, need_mask_pass ? ix.lay_r.ncb : 0u);
     g_launches++;
     if ((e = cudaGetLastError()) != cudaSuccess) return e;
@@ -1537,11 +1534,7 @@ static cudaError_t select_w(BitparIndex& ix, SelectLaunch& L, cudaEvent_t before
             L.host_score = nullptr;
         }
         if (L.ready_event) { // tell the caller that node_idx / score are final (the mask pass may still be running)
-            cudaStreamCaptureStatus cs = cudaStreamCaptureStatusNone;
-            if ((e = cudaStreamIsCapturing(bs, &cs)) != cudaSuccess) return e;
-            e = cudaEventRecordWithFlags(L.ready_event, bs,
-                                         cs == cudaStreamCaptureStatusActive ? cudaEventRecordExternal : cudaEventRecordDefault);
-            if (e != cudaSuccess) return e;
+            if ((e = record_ready_event(L.ready_event, bs)) != cudaSuccess) return e;
             L.ready_event = nullptr;
         }
         return cudaSuccess;

@@ -87,7 +87,7 @@ struct BitparIndex {
     uint32_t* rk_perm = nullptr;
     size_t cap_nodes = 0, cap_blobP = 0, cap_pods = 0;
     uint32_t N = 0, Nord = 0, W = 0, spl_stride = 1, n_spl = 0;
-    BitparLayout lay{}, layP{};
+    BitparLayout layP{};
     bool valid = false;
     int sms = 0;
     cudaStream_t aux = nullptr; // the argmax kernels run here, overlapped with k_mask_rows

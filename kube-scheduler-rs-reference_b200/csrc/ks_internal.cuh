@@ -150,4 +150,13 @@ struct SelectLaunch {
     PeerOut po;                        // fused all-gather of the bindings (po.n == 0: none)
 };
 
+// Records the caller's ready event on st.  Inside a stream capture it must become an external event node: a plain record
+// would only order nodes inside the graph and never signal the caller's event on replay.
+inline cudaError_t record_ready_event(cudaEvent_t ev, cudaStream_t st) {
+    cudaStreamCaptureStatus cs = cudaStreamCaptureStatusNone;
+    const cudaError_t e = cudaStreamIsCapturing(st, &cs);
+    if (e != cudaSuccess) return e;
+    return cudaEventRecordWithFlags(ev, st, cs == cudaStreamCaptureStatusActive ? cudaEventRecordExternal : cudaEventRecordDefault);
+}
+
 } // namespace ks
