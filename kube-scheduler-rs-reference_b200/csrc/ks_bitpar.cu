@@ -65,10 +65,7 @@ __device__ __forceinline__ bool key_less(int64_t av, uint32_t ai, int64_t bv, ui
 // KS_SCORE_LEAST_ALLOCATED bound: the score of node n for a pod that requests nothing.  For requests >= 0 the score of
 // every feasible (pod, n) cell is <= least_alloc_bound(n) (same truncating divisions, monotone in the numerators).
 __device__ __forceinline__ int64_t least_alloc_bound(const NodeTable& nt, uint32_t n) {
-    const int64_t fc = nt.free_cpu[n], fm = nt.free_mem[n], ac = nt.alloc_cpu[n], am = nt.alloc_mem[n];
-    const int64_t pc = ac > 0 ? (fc * 100) / ac : 0;
-    const int64_t pm = am > 0 ? (fm * 100) / am : 0;
-    return (pc + pm) / 2;
+    return least_alloc_score(nt.free_cpu[n], nt.free_mem[n], nt.alloc_cpu[n], nt.alloc_mem[n], 0, 0);
 }
 // prio[0..Npad) = leftover priority, prio[Npad..Npad+N) = least-allocated bound (k_node_bound, once per build)
 __device__ __forceinline__ int64_t order_value(const NodeTable& nt, const int64_t* __restrict__ prio, int k, uint32_t n) {
@@ -880,14 +877,9 @@ __device__ __forceinline__ void write_binding(const OutView& ov, const PodView& 
     int64_t score = 0;
     if (slot >= 0) {
         best = __ldg(ord_idx + slot);
-        score = __ldg(ord_prio + slot) - (int64_t)(((uint64_t)__ldg(pv.req_cpu + p) << 22) + (uint64_t)__ldg(pv.req_mem + p));
+        score = __ldg(ord_prio + slot) - leftover_cost(__ldg(pv.req_cpu + p), __ldg(pv.req_mem + p));
     }
-    if (ov.node_idx) ov.node_idx[p] = best;
-    if (ov.score) ov.score[p] = score;
-    for (uint32_t k = 0; k < po.n; k++) { // fused all-gather: the same binding goes to every peer over NVLink
-        po.idx[k][p] = best;
-        po.score[k][p] = score;
-    }
+    store_binding(ov, po, p, best, score);
 }
 
 constexpr uint32_t FF_HEAD_TILES = 2;
@@ -1040,8 +1032,8 @@ __device__ __forceinline__ int64_t div_floor_pos(int64_t x, int64_t d, double in
     return q;
 }
 
-// exactly the expression of k_select_direct / the oracle (truncating division; x may be negative only when the
-// request is negative, where the generic operator is used)
+// the same value as least_alloc_score(e.fc, e.fm, e.ac, e.am, rc, rm) (ks_internal.cuh), with the division by a
+// reciprocal (x may be negative only when the request is negative, where the generic operator is used)
 __device__ __forceinline__ int64_t least_alloc_score(const NodeEval& e, int64_t rc, int64_t rm) {
     int64_t pc = 0, pm = 0;
     if (e.ac > 0) {
@@ -1179,31 +1171,17 @@ __global__ void __launch_bounds__(256)
                     }
                 }
                 // every lane starts a tile with the same (best, bidx); merge only when some lane improved on it
-                if (__any_sync(0xffffffffu, changed)) {
-#pragma unroll
-                    for (int off = 16; off > 0; off >>= 1) { // every lane ends with the tile-merged best
-                        const int64_t os = __shfl_xor_sync(0xffffffffu, best, off);
-                        const int32_t oi = __shfl_xor_sync(0xffffffffu, bidx, off);
-                        if (oi >= 0 && (bidx < 0 || os > best || (os == best && oi < bidx))) {
-                            best = os;
-                            bidx = oi;
-                        }
-                    }
+                if (__any_sync(0xffffffffu, changed)) { // every lane ends with the tile-merged best
+                    const Candidate w = warp_argmax(best, bidx);
+                    best = w.key;
+                    bidx = w.idx;
                 }
             }
             __syncwarp(); // the next window overwrites this warp's slice of s_mask / s_top
             k0 += win;
             win = 32;
         }
-        if (lane == 0) {
-            const int64_t score = bidx >= 0 ? best : 0;
-            if (ov.node_idx) ov.node_idx[p] = bidx;
-            if (ov.score) ov.score[p] = score;
-            for (uint32_t q = 0; q < po.n; q++) {
-                po.idx[q][p] = bidx;
-                po.score[q][p] = score;
-            }
-        }
+        if (lane == 0) store_binding(ov, po, p, bidx, bidx >= 0 ? best : 0);
     }
     if (c_trace) {
         __syncthreads();

@@ -40,7 +40,7 @@ cudaError_t launch_free_reduce(int64_t* free_cpu, int64_t* free_mem, const int32
     return cudaGetLastError();
 }
 
-// range check of free values + static node priority for KS_SCORE_LEFTOVER: prio = free_cpu*2^22 + free_mem
+// range check of free values + static node priority for KS_SCORE_LEFTOVER (leftover_prio)
 __global__ void k_node_prio(const int64_t* __restrict__ free_cpu, const int64_t* __restrict__ free_mem,
                             int64_t* __restrict__ prio, uint32_t N, uint32_t Npad, int* __restrict__ range_flag) {
     uint32_t n = blockIdx.x * blockDim.x + threadIdx.x;
@@ -56,7 +56,7 @@ __global__ void k_node_prio(const int64_t* __restrict__ free_cpu, const int64_t*
         prio[n] = INT64_MIN + 1;
         return;
     }
-    prio[n] = fc * ((int64_t)1 << 22) + fm;
+    prio[n] = leftover_prio(fc, fm);
 }
 
 cudaError_t launch_node_prio(const int64_t* free_cpu, const int64_t* free_mem, int64_t* prio, uint32_t N,
@@ -72,14 +72,8 @@ cudaError_t launch_node_prio(const int64_t* free_cpu, const int64_t* free_mem, i
 __global__ void __launch_bounds__(256)
     k_exchange_push(PeerOut po, const int32_t* __restrict__ node_idx, const int64_t* __restrict__ score, uint32_t P) {
     if (blockIdx.x == 0 && threadIdx.x == 0) exchange_stamp(po, 0);
-    for (uint32_t p = blockIdx.x * blockDim.x + threadIdx.x; p < P; p += gridDim.x * blockDim.x) {
-        const int32_t ix = node_idx[p];
-        const int64_t sc = score[p];
-        for (uint32_t k = 0; k < po.n; k++) {
-            po.idx[k][p] = ix;
-            po.score[k][p] = sc;
-        }
-    }
+    for (uint32_t p = blockIdx.x * blockDim.x + threadIdx.x; p < P; p += gridDim.x * blockDim.x)
+        store_binding(OutView{}, po, p, node_idx[p], score[p]);
     exchange_signal(po);
 }
 
@@ -316,7 +310,7 @@ __global__ void __launch_bounds__(DIRECT_THREADS)
             const bool real = (uint32_t)node < nt.N; // padding sentinels are never feasible
             int64_t key_n = 0, ac = 0, am = 0;
             if (POLICY == KS_SCORE_LEFTOVER) {
-                key_n = (int64_t)(((uint64_t)fc << 22) + (uint64_t)fm); // node priority; pod part is constant
+                key_n = leftover_prio(fc, fm); // the pod part is constant
             } else {
                 ac = s_ac[ln];
                 am = s_am[ln];
@@ -331,6 +325,7 @@ __global__ void __launch_bounds__(DIRECT_THREADS)
                 const uint32_t b = __ballot_sync(0xffffffffu, ok);
                 cnt[i] += __popc(b);
                 if (EMIT_MASK) acc[i] = (lane == g) ? b : acc[i];
+                // ascending node per lane: strict '>' is argmax_better here, and cheaper
                 if (POLICY == KS_SCORE_LEFTOVER) {
                     if (ok && key_n > best[i]) {
                         best[i] = key_n;
@@ -338,9 +333,7 @@ __global__ void __launch_bounds__(DIRECT_THREADS)
                     }
                 } else {
                     if (ok) {
-                        int64_t pc = ac > 0 ? ((fc - rc[i]) * 100) / ac : 0;
-                        int64_t pm = am > 0 ? ((fm - rm[i]) * 100) / am : 0;
-                        int64_t s = (pc + pm) / 2;
+                        const int64_t s = least_alloc_score(fc, fm, ac, am, rc[i], rm[i]);
                         if (s > best[i]) {
                             best[i] = s;
                             bidx[i] = node;
@@ -360,41 +353,27 @@ __global__ void __launch_bounds__(DIRECT_THREADS)
         __syncthreads(); // everyone is done with `stage` before it is refilled two iterations later
     }
 
-    // warp argmax: larger key wins, ties -> lower node index
 #pragma unroll
     for (int i = 0; i < PW; i++) {
-        int64_t k = best[i];
-        int32_t ix = bidx[i];
-#pragma unroll
-        for (int off = 16; off > 0; off >>= 1) {
-            int64_t ok_ = __shfl_xor_sync(0xffffffffu, k, off);
-            int32_t oi = __shfl_xor_sync(0xffffffffu, ix, off);
-            bool take = (oi >= 0) && (ix < 0 || ok_ > k || (ok_ == k && oi < ix));
-            if (take) {
-                k = ok_;
-                ix = oi;
-            }
-        }
+        const Candidate w = warp_argmax(best[i], bidx[i]);
         if (lane == 0 && p0 + i < pv.P) {
             const uint32_t p = p0 + i;
             if (gridDim.y == 1) {
-                int64_t s = 0;
-                if (ix >= 0)
-                    s = (POLICY == KS_SCORE_LEFTOVER) ? k - (int64_t)(((uint64_t)rc[i] << 22) + (uint64_t)rm[i]) : k;
-                if (ov.node_idx) ov.node_idx[p] = ix;
+                const int64_t s = w.idx >= 0 ? key_to_score(POLICY, w.key, rc[i], rm[i]) : 0;
+                if (ov.node_idx) ov.node_idx[p] = w.idx;
                 if (ov.score) ov.score[p] = s;
                 if (ov.cnt) ov.cnt[p] = cnt[i];
             } else {
                 const uint64_t o = (uint64_t)blockIdx.y * pv.P + p;
-                part.key[o] = k;
-                part.idx[o] = ix;
+                part.key[o] = w.key;
+                part.idx[o] = w.idx;
                 part.cnt[o] = cnt[i];
             }
         }
     }
 }
 
-// combine partials of node chunks: ascending chunk order + strict '>' keeps the lowest node index on ties
+// combine partials of node chunks
 template <int POLICY>
 __global__ void k_select_combine(PodView pv, OutView ov, PartialView part, uint32_t n_chunks) {
     uint32_t p = blockIdx.x * blockDim.x + threadIdx.x;
@@ -407,16 +386,12 @@ __global__ void k_select_combine(PodView pv, OutView ov, PartialView part, uint3
         c += part.cnt[o];
         int32_t oi = part.idx[o];
         int64_t ok_ = part.key[o];
-        if (oi >= 0 && (ix < 0 || ok_ > k)) {
+        if (argmax_better(ok_, oi, k, ix)) {
             k = ok_;
             ix = oi;
         }
     }
-    int64_t s = 0;
-    if (ix >= 0)
-        s = (POLICY == KS_SCORE_LEFTOVER)
-                ? k - (int64_t)(((uint64_t)pv.req_cpu[p] << 22) + (uint64_t)pv.req_mem[p])
-                : k;
+    const int64_t s = ix >= 0 ? key_to_score(POLICY, k, pv.req_cpu[p], pv.req_mem[p]) : 0;
     if (ov.node_idx) ov.node_idx[p] = ix;
     if (ov.score) ov.score[p] = s;
     if (ov.cnt) ov.cnt[p] = c;

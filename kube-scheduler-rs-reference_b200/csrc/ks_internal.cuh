@@ -92,6 +92,120 @@ struct PartialView {
     uint32_t* cnt;
 };
 
+// ---- what a cell's result means ------------------------------------------------------------------------------------
+// The one device-side definition of the score policies (KS_SCORE_* in include/ksched.h), the argmax rule, claim
+// resolution and the binding store; oracle/oracle.c is the same definition on the CPU and the tests compare the two bit
+// for bit.  Feasibility is predicates.rs:42 (fit, non-strict) and :45-61 (selector); the reference itself has no score.
+// Free, allocatable and requested values are range-checked at snapshot time (KS_MAX_CPU_MILLI, KS_MAX_MEM_BYTES), so
+// no term below leaves int64.
+
+// KS_SCORE_LEFTOVER = leftover_prio(free) - leftover_cost(request): separable, so a node's rank does not depend on the
+// pod and the argmax keys are node priorities.  The unsigned shift is free_cpu * 2^22 without signed-overflow UB.
+__device__ __forceinline__ int64_t leftover_prio(int64_t fc, int64_t fm) {
+    return (int64_t)(((uint64_t)fc << 22) + (uint64_t)fm);
+}
+__device__ __forceinline__ int64_t leftover_cost(int64_t rc, int64_t rm) { return leftover_prio(rc, rm); }
+
+// KS_SCORE_LEAST_ALLOCATED: mean of the cpu and memory percentages left after the request, truncating divisions as in
+// C and Rust; a resource with allocatable <= 0 contributes 0.  Not separable: the argmax keys are the scores themselves.
+__device__ __forceinline__ int64_t least_alloc_score(int64_t fc, int64_t fm, int64_t ac, int64_t am, int64_t rc, int64_t rm) {
+    const int64_t pc = ac > 0 ? ((fc - rc) * 100) / ac : 0;
+    const int64_t pm = am > 0 ? ((fm - rm) * 100) / am : 0;
+    return (pc + pm) / 2;
+}
+
+// The score a binding reports for the winning argmax key of a pod with request (rc, rm).
+__device__ __forceinline__ int64_t key_to_score(int policy, int64_t key, int64_t rc, int64_t rm) {
+    return policy == KS_SCORE_LEFTOVER ? key - leftover_cost(rc, rm) : key;
+}
+
+// The argmax rule: the larger key wins, equal keys go to the lower node index; idx < 0 means "no feasible node" and
+// never wins.
+__device__ __forceinline__ bool argmax_better(int64_t key, int32_t idx, int64_t best_key, int32_t best_idx) {
+    return idx >= 0 && (best_idx < 0 || key > best_key || (key == best_key && idx < best_idx));
+}
+
+struct Candidate {
+    int64_t key;
+    int32_t idx;
+};
+
+// Merges the (key, idx) candidates of the 32 lanes by argmax_better; every lane gets the warp's winner.  Taken and
+// returned by value: reference parameters would make the caller's running best address-taken, and the compiler then
+// stops turning the caller's own compare-and-update into selects.
+__device__ __forceinline__ Candidate warp_argmax(int64_t key, int32_t idx) {
+#pragma unroll
+    for (int off = 16; off > 0; off >>= 1) {
+        const int64_t ok = __shfl_xor_sync(0xffffffffu, key, off);
+        const int32_t oi = __shfl_xor_sync(0xffffffffu, idx, off);
+        if (argmax_better(ok, oi, key, idx)) {
+            key = ok;
+            idx = oi;
+        }
+    }
+    return {key, idx};
+}
+
+// Claims against node capacity (streaming reconcile, include/ksched.h): the claims on one node are taken in arrival
+// order, each accepted iff its request still fits what the accepted claims before it left (predicates.rs:42), and the
+// accepted requests are committed to free[] (util.rs:31-36).  The caller has set keys[k] = node << 32 | k for every
+// claim k < n that names a node and keys[k] = ~0 for the others; keys must have room for n rounded up to a power of
+// two.  One CTA of THREADS threads (every thread calls this) sorts the keys (bitonic, shared memory), then one thread
+// per node segment walks it: a single writer per node, no atomics, deterministic.  request(k) returns claim k's (cpu,
+// memory); record(k, ok) is called once for every claim that names a node.  free[] is read through L2 because
+// k_stream_batch calls this after other CTAs of the same launch have written it.
+template <uint32_t THREADS, class Request, class Record>
+__device__ __forceinline__ void resolve_claims(unsigned long long* keys, uint32_t n, int64_t* free_cpu, int64_t* free_mem,
+                                               Request request, Record record) {
+    uint32_t m = 1;
+    while (m < n) m <<= 1;
+    for (uint32_t i = n + threadIdx.x; i < m; i += THREADS) keys[i] = ~0ull; // padding sorts last
+    __syncthreads();
+    for (uint32_t size = 2; size <= m; size <<= 1)
+        for (uint32_t stride = size >> 1; stride > 0; stride >>= 1) {
+            for (uint32_t i = threadIdx.x; i < m / 2; i += THREADS) {
+                const uint32_t lo = 2 * i - (i & (stride - 1)), hi = lo + stride;
+                const bool up = (lo & size) == 0;
+                const unsigned long long a = keys[lo], b = keys[hi];
+                if ((a > b) == up) {
+                    keys[lo] = b;
+                    keys[hi] = a;
+                }
+            }
+            __syncthreads();
+        }
+    for (uint32_t i = threadIdx.x; i < m; i += THREADS) {
+        const unsigned long long key = keys[i];
+        if (key == ~0ull) continue;
+        const uint32_t node = (uint32_t)(key >> 32);
+        if (i > 0 && (uint32_t)(keys[i - 1] >> 32) == node) continue; // not a segment head
+        int64_t fc = __ldcg(free_cpu + node), fm = __ldcg(free_mem + node);
+        for (uint32_t j = i; j < m && keys[j] != ~0ull && (uint32_t)(keys[j] >> 32) == node; j++) {
+            const uint32_t k = (uint32_t)keys[j];
+            const longlong2 r = request(k);
+            const bool ok = r.x <= fc && r.y <= fm;
+            record(k, ok);
+            if (ok) {
+                fc -= r.x;
+                fm -= r.y;
+            }
+        }
+        free_cpu[node] = fc;
+        free_mem[node] = fm;
+    }
+}
+
+// Stores pod p's binding into the local outputs the caller asked for and, with a fused exchange, into every peer's
+// gather buffer.
+__device__ __forceinline__ void store_binding(const OutView& ov, const PeerOut& po, uint32_t p, int32_t idx, int64_t score) {
+    if (ov.node_idx) ov.node_idx[p] = idx;
+    if (ov.score) ov.score[p] = score;
+    for (uint32_t k = 0; k < po.n; k++) {
+        po.idx[k][p] = idx;
+        po.score[k][p] = score;
+    }
+}
+
 extern std::atomic<uint64_t> g_launches;
 
 // ---- PTX helpers: mbarrier + 1-D TMA bulk copy (cp.async.bulk -> SASS UBLKCP) ----

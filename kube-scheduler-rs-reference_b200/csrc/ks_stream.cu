@@ -10,67 +10,30 @@ namespace cg = cooperative_groups;
 namespace ks {
 
 constexpr int STREAM_MAX = 4096; // claims per launch (one CTA sorts them in shared memory)
+constexpr uint32_t RESOLVE_THREADS = 1024;
 
-// One CTA.  (1) bitonic sort of (node, arrival) keys in shared memory; (2) one thread per node segment walks
-// its claimants in arrival order: accept iff the request still fits, then decrement free[] (single writer
-// per node: no atomics, deterministic).
-__global__ void __launch_bounds__(1024)
+// One CTA resolves the caller's claims (resolve_claims); a claim on a node outside [0, N) is rejected.
+__global__ void __launch_bounds__(RESOLVE_THREADS)
     k_stream_resolve(int64_t* __restrict__ free_cpu, int64_t* __restrict__ free_mem, const int32_t* __restrict__ claim_node,
                      const int64_t* __restrict__ req_cpu, const int64_t* __restrict__ req_mem, uint32_t n, uint32_t N,
                      uint8_t* __restrict__ accepted) {
     __shared__ unsigned long long key[STREAM_MAX];
-    uint32_t m = 1;
-    while (m < n) m <<= 1;
-    for (uint32_t i = threadIdx.x; i < m; i += blockDim.x) {
-        unsigned long long k = ~0ull; // padding and "no claim" sort last
-        if (i < n) {
-            const int32_t nd = claim_node[i];
-            if (nd >= 0 && (uint32_t)nd < N) k = ((unsigned long long)(uint32_t)nd << 32) | i;
-            else accepted[i] = 0;
-        }
-        key[i] = k;
+    for (uint32_t i = threadIdx.x; i < n; i += RESOLVE_THREADS) {
+        const int32_t nd = claim_node[i];
+        const bool valid = nd >= 0 && (uint32_t)nd < N;
+        if (!valid) accepted[i] = 0;
+        key[i] = valid ? ((unsigned long long)(uint32_t)nd << 32) | i : ~0ull;
     }
-    __syncthreads();
-    for (uint32_t size = 2; size <= m; size <<= 1) {
-        for (uint32_t stride = size >> 1; stride > 0; stride >>= 1) {
-            for (uint32_t i = threadIdx.x; i < m / 2; i += blockDim.x) {
-                const uint32_t lo = 2 * i - (i & (stride - 1)), hi = lo + stride;
-                const bool up = (lo & size) == 0;
-                const unsigned long long a = key[lo], b = key[hi];
-                if ((a > b) == up) {
-                    key[lo] = b;
-                    key[hi] = a;
-                }
-            }
-            __syncthreads();
-        }
-    }
-    for (uint32_t i = threadIdx.x; i < m; i += blockDim.x) {
-        const unsigned long long k = key[i];
-        if (k == ~0ull) continue;
-        const uint32_t node = (uint32_t)(k >> 32);
-        if (i > 0 && (uint32_t)(key[i - 1] >> 32) == node) continue; // not a segment head
-        int64_t fc = free_cpu[node], fm = free_mem[node];
-        for (uint32_t j = i; j < m && (uint32_t)(key[j] >> 32) == node && key[j] != ~0ull; j++) {
-            const uint32_t c = (uint32_t)key[j];
-            const int64_t rc = req_cpu[c], rm = req_mem[c];
-            const bool ok = rc <= fc && rm <= fm; // predicates.rs:42 against what is left
-            accepted[c] = ok;
-            if (ok) { // util.rs:31-36
-                fc -= rc;
-                fm -= rm;
-            }
-        }
-        free_cpu[node] = fc;
-        free_mem[node] = fm;
-    }
+    resolve_claims<RESOLVE_THREADS>(
+        key, n, free_cpu, free_mem, [&](uint32_t c) { return make_longlong2(req_cpu[c], req_mem[c]); },
+        [&](uint32_t c, bool ok) { accepted[c] = ok; });
 }
 
 cudaError_t launch_stream_resolve(int64_t* free_cpu, int64_t* free_mem, const int32_t* claim_node, const int64_t* req_cpu,
                                   const int64_t* req_mem, uint32_t n, uint32_t N, uint8_t* accepted, cudaStream_t st) {
     if (n == 0) return cudaSuccess;
     if (n > STREAM_MAX) return cudaErrorInvalidValue;
-    k_stream_resolve<<<1, 1024, 0, st>>>(free_cpu, free_mem, claim_node, req_cpu, req_mem, n, N, accepted);
+    k_stream_resolve<<<1, RESOLVE_THREADS, 0, st>>>(free_cpu, free_mem, claim_node, req_cpu, req_mem, n, N, accepted);
     g_launches++;
     return cudaGetLastError();
 }
@@ -83,7 +46,7 @@ uint32_t stream_max_claims() { return STREAM_MAX; }
 //   A  every CTA scans its slice of the node table for every pending pod (one warp per pod, lanes over nodes):
 //      feasible (predicates.rs:42,45-61) -> policy key -> warp argmax (ties -> lowest node index) -> partial[pod][cta]
 //   B  CTA 0 reduces the partials to one claim per pod, resolves the claims per node in arrival order against what
-//      is left (same walk as k_stream_resolve), commits the accepted requests to free[], writes the bindings and
+//      is left (resolve_claims, as k_stream_resolve), commits the accepted requests to free[], writes the bindings and
 //      compacts the losers (order preserved) into the next round's pending list
 // separated by grid-wide barriers.  Batches of up to STREAM_BATCH_MAX pods.
 constexpr uint32_t SB_THREADS = 256;
@@ -136,33 +99,19 @@ __global__ void __launch_bounds__(SB_THREADS)
 #pragma unroll
                 for (int w = 0; w < W; w++) miss |= sw[w] & ~labels[(size_t)w * Npad + n];
                 if (rc <= fc && rm <= fm && miss == 0) {
-                    int64_t key;
-                    if (policy == KS_SCORE_LEFTOVER) {
-                        key = (int64_t)(((uint64_t)fc << 22) + (uint64_t)fm);
-                    } else {
-                        const int64_t ac = alloc_cpu[n], am = alloc_mem[n];
-                        const int64_t pc = ac > 0 ? ((fc - rc) * 100) / ac : 0;
-                        const int64_t pm = am > 0 ? ((fm - rm) * 100) / am : 0;
-                        key = (pc + pm) / 2;
-                    }
-                    if (key > best) { // ascending n per lane: strict '>' keeps the lowest index
+                    const int64_t key = policy == KS_SCORE_LEFTOVER
+                                            ? leftover_prio(fc, fm)
+                                            : least_alloc_score(fc, fm, alloc_cpu[n], alloc_mem[n], rc, rm);
+                    if (key > best) { // ascending n per lane: strict '>' is argmax_better here, and cheaper
                         best = key;
                         bidx = (int32_t)n;
                     }
                 }
             }
-#pragma unroll
-            for (int off = 16; off > 0; off >>= 1) {
-                const int64_t ok_ = __shfl_xor_sync(0xffffffffu, best, off);
-                const int32_t oi = __shfl_xor_sync(0xffffffffu, bidx, off);
-                if (oi >= 0 && (bidx < 0 || ok_ > best || (ok_ == best && oi < bidx))) {
-                    best = ok_;
-                    bidx = oi;
-                }
-            }
+            const Candidate w = warp_argmax(best, bidx);
             if (lane == 0) {
-                pkey[(size_t)k * G + blockIdx.x] = best;
-                pidx[(size_t)k * G + blockIdx.x] = bidx;
+                pkey[(size_t)k * G + blockIdx.x] = w.key;
+                pidx[(size_t)k * G + blockIdx.x] = w.idx;
             }
         }
         __threadfence();
@@ -175,71 +124,30 @@ __global__ void __launch_bounds__(SB_THREADS)
                 for (uint32_t c = lane; c < G; c += 32) { // ascending CTA = ascending node range
                     const int64_t ok_ = __ldcg(pkey + (size_t)k * G + c);
                     const int32_t oi = __ldcg(pidx + (size_t)k * G + c);
-                    if (oi >= 0 && (bidx < 0 || ok_ > best)) {
+                    if (argmax_better(ok_, oi, best, bidx)) {
                         best = ok_;
                         bidx = oi;
                     }
                 }
-#pragma unroll
-                for (int off = 16; off > 0; off >>= 1) {
-                    const int64_t ok_ = __shfl_xor_sync(0xffffffffu, best, off);
-                    const int32_t oi = __shfl_xor_sync(0xffffffffu, bidx, off);
-                    if (oi >= 0 && (bidx < 0 || ok_ > best || (ok_ == best && oi < bidx))) {
-                        best = ok_;
-                        bidx = oi;
-                    }
-                }
+                const Candidate w = warp_argmax(best, bidx);
                 if (lane == 0) {
-                    s_claim[k] = bidx;
-                    s_ckey[k] = best;
+                    s_claim[k] = w.idx;
+                    s_ckey[k] = w.key;
                 }
             }
             __syncthreads();
-            // claims per node in arrival (batch) order: sort (node, k), one thread per node segment walks it
-            uint32_t m2 = 1;
-            while (m2 < cnt) m2 <<= 1;
-            for (uint32_t i = tid; i < m2; i += SB_THREADS) {
-                unsigned long long key = ~0ull;
-                if (i < cnt) {
-                    s_acc[i] = 0;
-                    if (s_claim[i] >= 0) key = ((unsigned long long)(uint32_t)s_claim[i] << 32) | i;
-                }
-                s_key[i] = key;
+            // claims per node in arrival (batch) order
+            for (uint32_t i = tid; i < cnt; i += SB_THREADS) {
+                s_acc[i] = 0;
+                s_key[i] = s_claim[i] >= 0 ? ((unsigned long long)(uint32_t)s_claim[i] << 32) | i : ~0ull;
             }
-            __syncthreads();
-            for (uint32_t size = 2; size <= m2; size <<= 1)
-                for (uint32_t stride = size >> 1; stride > 0; stride >>= 1) {
-                    for (uint32_t i = tid; i < m2 / 2; i += SB_THREADS) {
-                        const uint32_t lo = 2 * i - (i & (stride - 1)), hi = lo + stride;
-                        const bool up = (lo & size) == 0;
-                        const unsigned long long a = s_key[lo], b = s_key[hi];
-                        if ((a > b) == up) {
-                            s_key[lo] = b;
-                            s_key[hi] = a;
-                        }
-                    }
-                    __syncthreads();
-                }
-            for (uint32_t i = tid; i < m2; i += SB_THREADS) {
-                const unsigned long long key = s_key[i];
-                if (key == ~0ull) continue;
-                const uint32_t node = (uint32_t)(key >> 32);
-                if (i > 0 && (uint32_t)(s_key[i - 1] >> 32) == node) continue; // not a segment head
-                int64_t fc = __ldcg(free_cpu + node), fm = __ldcg(free_mem + node);
-                for (uint32_t j = i; j < m2 && s_key[j] != ~0ull && (uint32_t)(s_key[j] >> 32) == node; j++) {
-                    const uint32_t k = (uint32_t)s_key[j];
+            resolve_claims<SB_THREADS>(
+                s_key, cnt, free_cpu, free_mem,
+                [&](uint32_t k) {
                     const uint32_t p = __ldcg(pl + k);
-                    const int64_t rc = req_cpu[p], rm = req_mem[p];
-                    const bool ok = rc <= fc && rm <= fm; // predicates.rs:42 against what is left
-                    s_acc[k] = ok;
-                    if (ok) { // util.rs:31-36
-                        fc -= rc;
-                        fm -= rm;
-                    }
-                }
-                free_cpu[node] = fc;
-                free_mem[node] = fm;
-            }
+                    return make_longlong2(req_cpu[p], req_mem[p]);
+                },
+                [&](uint32_t k, bool ok) { s_acc[k] = ok; });
             __syncthreads();
             // bindings of the winners; losers keep their order in the next pending list
             uint32_t* nl = pend + (cur ^ 1u) * STREAM_BATCH_MAX;
@@ -253,9 +161,7 @@ __global__ void __launch_bounds__(SB_THREADS)
                     const uint32_t p = __ldcg(pl + k);
                     if (s_acc[k]) {
                         out_idx[p] = s_claim[k];
-                        out_score[p] = policy == KS_SCORE_LEFTOVER
-                                           ? s_ckey[k] - (int64_t)(((uint64_t)req_cpu[p] << 22) + (uint64_t)req_mem[p])
-                                           : s_ckey[k];
+                        out_score[p] = key_to_score(policy, s_ckey[k], req_cpu[p], req_mem[p]);
                     } else {
                         loser[e] = 1;
                         n_loser++;

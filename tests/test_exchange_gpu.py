@@ -15,7 +15,7 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 pytestmark = pytest.mark.gpu
 
 
-def _worker(rank, world, port, P, N, flags, steps, q):
+def _worker(rank, world, port, P, N, flags, steps, policy, q):
     try:
         sys.path.insert(0, ROOT)
         import torch
@@ -51,12 +51,12 @@ def _worker(rank, world, port, P, N, flags, steps, q):
             torch.cuda.synchronize()
             dist.barrier()  # nobody overwrites a gather buffer that a peer is still reading
             snap.select_raw(n, t[0], t[1], t[2], ks.KS_MEM_DEVICE, xch.node_idx_ptr, xch.score_ptr, cnt, ks.KS_MEM_DEVICE,
-                            mask=mask, mask_row_bytes=row, mask_space=ks.KS_MEM_DEVICE, flags=flags, stream=st.cuda_stream,
-                            exchange=xch)
+                            mask=mask, mask_row_bytes=row, mask_space=ks.KS_MEM_DEVICE, policy=policy, flags=flags,
+                            stream=st.cuda_stream, exchange=xch)
             st.synchronize()
             snap.exchange_check()
             g_idx, g_score = xch.read()
-            fi, fs, fcn, fmask, _ = orc.run_packed(fc, fm, ac, am, lab, rc_it, rm, sel, want_mask=True, nthreads=2 if P * N < 10**9 else 16)
+            fi, fs, fcn, fmask, _ = orc.run_packed(fc, fm, ac, am, lab, rc_it, rm, sel, policy=policy, want_mask=True, nthreads=2 if P * N < 10**9 else 16)
             for r in range(world):
                 l, h = ks.multigpu.shard_bounds(P, world, r)
                 ok &= np.array_equal(g_idx[r, :h - l], fi[l:h]) and np.array_equal(g_score[r, :h - l], fs[l:h])
@@ -72,16 +72,19 @@ def _worker(rank, world, port, P, N, flags, steps, q):
         q.put((rank, False, -1, traceback.format_exc()[-1500:] + str(e)))
 
 
-@pytest.mark.parametrize("P,N,flags,steps", [(40000, 3000, 2, 3), (3001, 2500, 1, 3), (1, 5000, 2, 3), (90000, 50000, 2, 1)])
-def test_fused_exchange_two_ranks(P, N, flags, steps):
+@pytest.mark.parametrize("P,N,flags,steps,policy", [
+    (40000, 3000, 2, 3, 0), (3001, 2500, 1, 3, 0), (1, 5000, 2, 3, 0), (90000, 50000, 2, 1, 0), (40000, 3000, 2, 3, 1)],
+    ids=["40000-3000-2-3", "3001-2500-1-3", "1-5000-2-3", "90000-50000-2-1", "40000-3000-2-3-least_allocated"])
+def test_fused_exchange_two_ranks(P, N, flags, steps, policy):
     """flags 2 = bit-parallel path (stores fused into the argmax kernels), 1 = per-cell path (push kernel);
+    policy 1 = KS_SCORE_LEAST_ALLOCATED, whose bit-parallel argmax kernel (k_least_alloc) stores to the peers itself;
     P = 1 leaves rank 1 with an empty shard; 90000 x 50000 is a long mask pass (282 MB per rank): 896-thread mask CTAs with
     128-thread argmax CTAs beside them, where the small cases run the argmax kernels on SMs the mask kernel leaves free."""
     import torch.multiprocessing as mp
     ctx = mp.get_context("spawn")
     q = ctx.Queue()
     port = 32000 + (os.getpid() % 2000) + flags
-    procs = [ctx.Process(target=_worker, args=(r, 2, port, P, N, flags, steps, q)) for r in range(2)]
+    procs = [ctx.Process(target=_worker, args=(r, 2, port, P, N, flags, steps, policy, q)) for r in range(2)]
     for p in procs:
         p.start()
     res = [q.get(timeout=600) for _ in procs]
